@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Learner throughput benchmark (BASELINE.json metric: learner sequences/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--channels C] [--fast] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--channels C] [--fast] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one learner update on one batch of 64 replay sequences (b/l/f = 40/40/5 -> 85 frames
 of C x 84 x 84 u8 each):
@@ -384,6 +384,18 @@ def run_ingest_mode(args, learner, replay, C, ms_step_plain):
                     "into pinned memory by the prefetch thread and copied on the ingest stream while the previous update runs"}
 
 
+def last_update_outputs(learner, replay) -> dict:
+    """What the replay update path leaves its caller after an update: that update's TD errors, priorities, Q values and
+    loss, the online parameters after its optimizer step, and the sum tree's leaves after its priority update."""
+    core, tree = learner.core, replay.tree
+    torch.cuda.synchronize()
+    rows = int(core.rows.item())
+    leaf0 = tree.num_nodes // 2
+    out = {"td": core.td[:rows], "priorities": core.prio, "q": core.q[:rows], "loss": core.loss_sum.double() / rows,
+           "online_params": core.online.flat, "tree_leaves": tree.nodes_device()[leaf0:leaf0 + tree.capacity]}
+    return {k: v.cpu().numpy() for k, v in out.items()}
+
+
 def run_ours(args):
     import torch.distributed as dist
     from r2d2_b200 import _lib, config
@@ -493,6 +505,7 @@ def run_ours(args):
         for w in range(6):                                            # untimed: the second set of batch buffers gets its CUDA graph
             step_resident(w)                                          # (a key is captured the second time it is seen)
     ms_step = timed(step_resident, args.steps, args.warmup)
+    outputs = last_update_outputs(learner, replay) if args.dump_outputs and rank == 0 else None
     ms_e2e = timed(step_e2e, args.steps, args.warmup)
     sampler.stop_flag = True
 
@@ -587,6 +600,10 @@ def run_ours(args):
                 line["vs_cuda_eager"] = {"reference_value": eager["value"], "unit": "sequences/s", "ratio": value / eager["value"],
                                          "e2e_ratio": e2e / eager["value"], "sample": eager["cpu_baseline"]["sample"],
                                          "ms_per_step": eager["ms_per_step"]}
+        if outputs is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in outputs.items():
+                np.save(os.path.join(args.dump_outputs, f"{name}.npy"), arr)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -614,6 +631,10 @@ def main():
                     help="time the strictly sequential loop only (default: batch i+1 is sampled and gathered while update i runs)")
     ap.add_argument("--timeline", action="store_true", help="also write gpurun_out/timeline_n<N>.txt (chronological device activities of 3 steps; ranks 0 and 1)")
     ap.add_argument("--kernel-times", action="store_true", help="also write gpurun_out/kernel_times.txt (per-kernel CUPTI durations)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed replay update computed (td, priorities, q, loss, online_params, tree_leaves) "
+                         "as DIR/<name>.npy, float32 or float64, about 25 MB; inputs are seeded, so runs with the same arguments "
+                         "can be compared output for output")
     args = ap.parse_args()
     # more hardware work queues than the default 8: the staging copies of the next batch must never share a queue with (and so
     # wait behind) the CUDA graph of the running update.  Must be set before CUDA is initialised.

@@ -10,6 +10,8 @@ fixtures hold only small side arrays and the reference's OUTPUTS):
                       indices, zero priorities, an empty update and a
                       non-power-of-two capacity; the full tree after every op,
                       sampled indices and IS weights.
+  tree_large.npz      the same class at 50,000 and 2^16 leaves: two rounds of
+                      sample() + update() of the sampled leaves per capacity.
   replay_ragged.npz   ``LocalBuffer.finish`` -> ``ReplayBuffer.add`` ->
                       ``sample_batch`` / ``update_priorities`` (worker.py:141-261,
                       437-497) on the ragged episode script: per-block metadata,
@@ -81,6 +83,37 @@ def gen_tree(ref):
                 out[f"{tag}_op{k}_isw"] = w.copy()
     np.savez_compressed(os.path.join(OUT, "tree_small.npz"), **out)
     print("tree_small.npz", len(out), "arrays")
+
+
+def tree_large_script():
+    """Per capacity: every leaf's TD error, then two rounds of (n, TD errors written to the n leaves sampled with
+    np.random.seed(n))."""
+    rng = np.random.default_rng(0)
+    cases = []
+    for cap in (50_000, 1 << 16):
+        td = rng.uniform(1e-3, 1, cap).astype(np.float32)
+        cases.append((cap, td, [(n, rng.uniform(0, 2, n).astype(np.float32)) for n in (64, 4096)]))
+    return cases
+
+
+def gen_tree_large(ref):
+    """Sampled indices and IS weights of every round, and the tree after its update: a CRC of the whole node array
+    plus 2048 nodes at seeded positions (the full trees would be 2 MB)."""
+    out = {}
+    for cap, td, rounds in tree_large_script():
+        tree = ref.priority_tree.PriorityTree(cap, 0.9, 0.6)
+        tree.update(np.arange(cap), td)
+        pos = np.sort(np.random.default_rng(cap).choice(tree.ptree.size, 2048, replace=False))
+        for n, t2 in rounds:
+            np.random.seed(n)
+            idx, w = tree.sample(n)
+            tree.update(idx, t2)
+            tag = f"c{cap}_n{n}"
+            out[f"{tag}_idx"], out[f"{tag}_isw"] = idx.copy(), w.copy()
+            out[f"{tag}_tree_crc"] = np.int64(crc(tree.ptree))
+            out[f"{tag}_tree_pos"], out[f"{tag}_tree_sample"] = pos, tree.ptree[pos].copy()
+    np.savez_compressed(os.path.join(OUT, "tree_large.npz"), **out)
+    print("tree_large.npz", len(out), "arrays")
 
 
 # ------------------------------------------------------------------------------ replay + learner
@@ -242,6 +275,7 @@ def main():
     torch.set_num_threads(8)
     ref = ref_harness.load()
     gen_tree(ref)
+    gen_tree_large(ref)
     gen_replay(ref)
     gen_learner(ref, "learner_ragged.npz", synth.RAGGED_SCRIPT, 8, 8, 3, 400, 40, 40, 5, seed0=40)
     gen_learner(ref, "learner_cfg0.npz", CFG0_SCRIPT, 8, 4, 2, 40, 8, 8, 4, seed0=60)

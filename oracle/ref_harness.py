@@ -2,8 +2,8 @@
 
 The reference is read from /root/reference in the build container and from
 ``baseline/_ref`` (a verbatim, git-ignored copy made by ``__graft_entry__.build()``)
-on the GPU box.  Used by ``oracle/gen_golden.py``, by tests (skipped when neither
-directory exists) and by ``bench.py --impl reference``.  Two shims, both described in SURVEY.md section 8(c):
+on the GPU box.  Used by ``oracle/gen_golden.py``, which records the reference's
+outputs under tests/golden, and by ``bench.py --impl reference``.  Two shims, both described in SURVEY.md section 8(c):
 
   * a stub ``gym`` module (``environment.py`` imports gym at module level; only
     ``gym.Wrapper``, ``gym.ObservationWrapper``, ``gym.spaces.Box`` and

@@ -80,6 +80,27 @@ def test_dropin_modules_alias_the_package():
             sys.modules.pop(name, None)
 
 
+def test_dropin_config_overrides_in_a_fresh_process(tmp_path):
+    """With dropin/ on PYTHONPATH, a script's `import config` binds this package's config with R2D2_CONFIG_OVERRIDES
+    applied before `worker` captures its def-time defaults; an unknown name is an error."""
+    import json
+    import subprocess
+    import sys
+    code = ("import config, worker, r2d2_b200.config as pkg\n"
+            "from worker import Learner, Actor, ReplayBuffer\n"
+            "assert config is pkg\n"
+            "print(config.training_steps, config.batch_size, config.seq_len, worker.Learner.__init__.__defaults__[3])\n")
+    env = dict(os.environ)
+    env["PYTHONPATH"] = os.pathsep.join([os.path.join(ROOT, "dropin"), ROOT, env.get("PYTHONPATH", "")])
+    env["R2D2_CONFIG_OVERRIDES"] = json.dumps({"training_steps": 6, "batch_size": 8, "learning_steps": 10, "game_name": "Pong"})
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300, cwd=str(tmp_path), env=env)
+    assert r.returncode == 0, r.stderr[-3000:]
+    assert r.stdout.split() == ["6", "8", "55", "Pong"], r.stdout
+    env["R2D2_CONFIG_OVERRIDES"] = json.dumps({"trainig_steps": 6})
+    r = subprocess.run([sys.executable, "-c", "import config"], capture_output=True, text=True, timeout=300, cwd=str(tmp_path), env=env)
+    assert r.returncode != 0 and "unknown config name 'trainig_steps'" in r.stderr, r.stderr[-3000:]
+
+
 def test_local_buffer_blocks_match_reference_golden(golden_dir):
     """The product's host-side block cutter (worker.LocalBuffer) against the reference's recorded blocks."""
     from r2d2_b200.worker import LocalBuffer

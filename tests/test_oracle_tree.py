@@ -4,9 +4,8 @@ import os
 import numpy as np
 import pytest
 
-from oracle.gen_golden import tree_script
+from oracle.gen_golden import crc, tree_large_script, tree_script
 from oracle.sumtree import SumTreeOracle
-from oracle import ref_harness
 
 
 @pytest.mark.parametrize("tag,cap", [("p2", 1024), ("np2", 1000), ("tiny", 3)])
@@ -26,23 +25,17 @@ def test_tree_matches_reference_golden(golden_dir, tag, cap):
             np.testing.assert_array_equal(w, g[f"{tag}_op{k}_isw"])
 
 
-@pytest.mark.skipif(not ref_harness.available(), reason="reference not present on this box")
-def test_tree_live_against_reference_large():
-    ref = ref_harness.load()
-    rng = np.random.default_rng(0)
-    for cap in (50_000, 1 << 16):
-        a = ref.priority_tree.PriorityTree(cap, 0.9, 0.6)
-        b = SumTreeOracle(cap, 0.9, 0.6)
-        td = rng.uniform(1e-3, 1, cap).astype(np.float32)
-        a.update(np.arange(cap), td)
-        b.update(np.arange(cap), td)
-        for n in (64, 4096):
-            np.random.seed(n)
-            ia, wa = a.sample(n)
-            ib, wb = b.sample(n, np.random.RandomState(n).random_sample(n))
-            np.testing.assert_array_equal(ia, ib)
-            np.testing.assert_array_equal(wa, wb)
-            t2 = rng.uniform(0, 2, n).astype(np.float32)
-            a.update(ia, t2)
-            b.update(ib, t2)
-            np.testing.assert_array_equal(a.ptree, b.ptree)
+def test_tree_matches_reference_golden_large(golden_dir):
+    """50,000 and 2^16 leaves: sampled indices, IS weights and the whole tree (CRC) after each round, bit-exact."""
+    g = np.load(os.path.join(golden_dir, "tree_large.npz"))
+    for cap, td, rounds in tree_large_script():
+        tree = SumTreeOracle(cap, 0.9, 0.6)
+        tree.update(np.arange(cap), td)
+        for n, t2 in rounds:
+            tag = f"c{cap}_n{n}"
+            idx, w = tree.sample(n, np.random.RandomState(n).random_sample(n))
+            np.testing.assert_array_equal(idx, g[f"{tag}_idx"])
+            np.testing.assert_array_equal(w, g[f"{tag}_isw"])
+            tree.update(idx, t2)
+            np.testing.assert_array_equal(tree.ptree[g[f"{tag}_tree_pos"]], g[f"{tag}_tree_sample"])
+            assert crc(tree.ptree) == int(g[f"{tag}_tree_crc"])
